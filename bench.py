@@ -300,7 +300,7 @@ def run_tiled(args, wl, name, gb, dist, rank, world, local, steps, warmup):
             ok, jpeg = gb.process(params, st, rgb, w, h, device=local)
         if not ok:
             raise RuntimeError("tiled Process failed: " + gb.last_error())
-        return st, hashlib.sha256(jpeg).hexdigest()
+        return st, jpeg
 
     for _ in range(warmup):
         once()
@@ -308,10 +308,10 @@ def run_tiled(args, wl, name, gb, dist, rank, world, local, steps, warmup):
     tm = DeviceTimer()
     tm.start()
     shas = set()
-    st = None
+    st = jpeg = None
     for _ in range(steps):
-        st, sha = once()
-        shas.add(sha)
+        st, jpeg = once()
+        shas.add(hashlib.sha256(jpeg).hexdigest())
     dt_local = tm.stop()
     gdist.barrier(dist, cuda=HAVE_CUDA)
     dt = gdist.max_over_ranks(dist, dt_local, device=f"cuda:{local}" if HAVE_CUDA else None)
@@ -328,7 +328,22 @@ def run_tiled(args, wl, name, gb, dist, rank, world, local, steps, warmup):
            "iterations": st.counters["number of iterations"]}
     if world > 1:
         gb.dist_shutdown()
-    return out
+    return out, jpeg
+
+
+def dump_outputs(path, jpegs, rank, world, budget=64 << 20):
+    """What the timed path returned in its last step: every JPEG file as DIR/jpeg_<image>.npy, its
+    bytes as float32, at most `budget` bytes over all ranks.  A JPEG larger than its share is stored
+    as a fixed sample of its bytes (positions drawn with seed 0, in increasing order, the same for
+    equal file sizes); DIR/sizes_rank<r>.npy holds the full sizes of rank r's files."""
+    os.makedirs(path, exist_ok=True)
+    share = max(1, (budget - 4096 * world) // 4 // (world * len(jpegs)))
+    for i, data in jpegs.items():
+        a = np.frombuffer(data, dtype=np.uint8)
+        if a.size > share:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, share, replace=False))]
+        np.save(os.path.join(path, "jpeg_%03d.npy" % i), a.astype(np.float32))
+    np.save(os.path.join(path, "sizes_rank%d.npy" % rank), np.array([len(d) for d in jpegs.values()], dtype=np.float64))
 
 
 def claim_stdout():
@@ -363,6 +378,8 @@ def main():
                     help="skip the extra 8K image tiled over all ranks at the end of a batch-mode run")
     ap.add_argument("--tiled-leg-workload", default="gradnoise8k_q95", choices=sorted(WORKLOADS))
     ap.add_argument("--tiled-leg-timeout", type=float, default=900.0)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the JPEGs of the last step to DIR as .npy (float32) files")
     args = ap.parse_args()
     wl = WORKLOADS[args.workload]
 
@@ -394,9 +411,11 @@ def main():
         sampler = ClockSampler(local)
         sampler.start()
         n0, a0, b0 = gb.counters()
-        res = run_tiled(args, wl, args.workload, gb, dist, rank, world, local, args.steps, args.warmup)
+        res, jpeg = run_tiled(args, wl, args.workload, gb, dist, rank, world, local, args.steps, args.warmup)
         n1, a1, b1 = gb.counters()
         clocks = sampler.stop()
+        if args.dump_outputs and rank == 0:  # every rank holds the same file
+            dump_outputs(args.dump_outputs, {0: jpeg}, 0, 1)
         if dist is not None:
             dist.destroy_process_group()
         if rank != 0:
@@ -424,6 +443,7 @@ def main():
     px = h * w
     pool = ThreadPoolExecutor(M)
     shas = [set() for _ in range(M)]
+    last = {}  # image index -> JPEG of the latest timed step
 
     def encode_host(j):  # reference-facing call: host buffer in, JPEG bytes out
         st = gb.ProcessStats()
@@ -443,6 +463,7 @@ def main():
         if not ok:
             raise RuntimeError(f"gb200_image_process failed on image {j}: {gb.last_error()}")
         shas[j].add(hashlib.sha256(jpeg).hexdigest())
+        last[rank * M + j] = jpeg
         return st
 
     for _ in range(args.warmup):
@@ -469,6 +490,8 @@ def main():
         img.close()
     resident.clear()
     value = world * args.steps * M * px / dt / 1e6
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(sorted(last.items())), rank, world)
 
     # ---- e2e: same job through the reference-facing call with HOST buffers ----
     gdist.barrier(dist, cuda=HAVE_CUDA)
@@ -523,7 +546,7 @@ def main():
         def leg():
             try:
                 box["res"] = run_tiled(args, WORKLOADS[args.tiled_leg_workload], args.tiled_leg_workload, gb, dist,
-                                       rank, world, local, steps=1, warmup=0)
+                                       rank, world, local, steps=1, warmup=0)[0]
             except Exception as e:  # the main line must survive a failure of the extra leg
                 box["res"] = {"error": f"{type(e).__name__}: {e}"}
 

@@ -34,7 +34,13 @@ def target_for_quality(q):
     return float(np.float32(lib().gref_target_for_quality(float(q))))
 
 
-def process_rgb(rgb, quality=95.0, trace=True, lookahead=3, new_zeroing_model=True):
+def score_for_quality(q):
+    """ButteraugliScoreForQuality in double precision (target_for_quality narrows it to float)."""
+    return lib().gref_target_for_quality(float(q))
+
+
+def process_rgb(rgb, quality=95.0, trace=True, lookahead=3, new_zeroing_model=True, try_420=False, force_420=False,
+                clear_metadata=True):
     """-> (ok, jpeg bytes, trace str, counters[3], seconds)"""
     rgb = np.ascontiguousarray(rgb, dtype=np.uint8)
     h, w, _ = rgb.shape
@@ -44,10 +50,16 @@ def process_rgb(rgb, quality=95.0, trace=True, lookahead=3, new_zeroing_model=Tr
     tr_len = C.c_size_t()
     counters = (C.c_int * 3)()
     secs = C.c_double()
-    ok = lib().gref_process_rgb_ex(
-        _p(rgb, C.c_uint8), w, h, C.c_float(target_for_quality(quality)), int(lookahead), int(new_zeroing_model),
-        C.byref(out), C.byref(out_len),
-        C.byref(tr) if trace else None, C.byref(tr_len), counters, C.byref(secs))
+    lib().gref_set_420(int(try_420), int(force_420))
+    lib().gref_set_clear_metadata(int(clear_metadata))
+    try:
+        ok = lib().gref_process_rgb_ex(
+            _p(rgb, C.c_uint8), w, h, C.c_float(target_for_quality(quality)), int(lookahead), int(new_zeroing_model),
+            C.byref(out), C.byref(out_len),
+            C.byref(tr) if trace else None, C.byref(tr_len), counters, C.byref(secs))
+    finally:
+        lib().gref_set_420(0, 0)
+        lib().gref_set_clear_metadata(1)
     data = C.string_at(out, out_len.value)
     lib().gref_free(out)
     t = ""
@@ -208,6 +220,31 @@ def block_mask(rgb):
     h, w, _ = rgb.shape
     out = np.zeros((3, h, w), dtype=np.float32)
     lib().gref_block_mask(_p(rgb, C.c_uint8), w, h, _p(out, C.c_float))
+    return out
+
+
+def block_corner_mask(rgb):
+    """block_mask at the top-left pixel of every 8x8 block -> [nblocks][3]"""
+    m = block_mask(rgb)
+    return np.stack([m[c][::8, ::8].reshape(-1) for c in range(3)], axis=1)
+
+
+def heatmap(distmap):
+    """butteraugli_main's CreateHeatMapImage of a [h][w] diffmap -> [h][w][3] uint8"""
+    d = np.ascontiguousarray(distmap, dtype=np.float32)
+    h, w = d.shape
+    out = np.zeros((h, w, 3), dtype=np.uint8)
+    lib().gref_heatmap(_p(d, C.c_float), w, h, _p(out, C.c_uint8))
+    return out
+
+
+def huffman_depths(counts, limits):
+    """CreateHuffmanTree's code lengths for every row of counts [t][n] with the length limit limits[t]"""
+    counts = np.ascontiguousarray(counts, dtype=np.uint32)
+    t, n = counts.shape
+    out = np.zeros((t, n), dtype=np.uint8)
+    for i in range(t):
+        lib().gref_huffman_depths(_p(counts[i], C.c_uint32), n, int(limits[i]), _p(out[i], C.c_uint8))
     return out
 
 

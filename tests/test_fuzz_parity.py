@@ -13,12 +13,12 @@ _spec.loader.exec_module(fuzz)
 
 @pytest.mark.parametrize("seed", [3, 11, 19, 24, 30, 37, 1012, 2044])
 def test_random_case_matches_reference(port_lib, ref, seed):
-    same, info = fuzz.one(seed, port_lib)
+    same, info = fuzz.one(seed, port_lib, ref)
     assert same, info
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("seed", [3, 19, 30, 1012])
 def test_random_case_matches_reference_cuda(cuda_lib, ref, seed):
-    same, info = fuzz.one(seed, cuda_lib)
+    same, info = fuzz.one(seed, cuda_lib, ref)
     assert same, info

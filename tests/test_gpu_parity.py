@@ -1,5 +1,5 @@
 """GPU suite (-m gpu): the CUDA product, through its C ABI, against the oracle
-(the real reference build oracle/_ref, prebuilt and shipped with the snapshot)
+(the unmodified reference, as its recorded answers: tests/refanswers.py)
 and the committed golden answers.  Bit-exact everywhere: integers, float bit
 patterns of every butteraugli stage, JPEG bytes and the verbose trace."""
 import numpy as np

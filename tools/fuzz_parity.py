@@ -42,13 +42,13 @@ def random_image(rng):
     return np.clip(np.round(img), 0, 255).astype(np.uint8), kind
 
 
-def one(seed, port):
+def one(seed, port, ref=reflib):
     rng = np.random.default_rng(seed)
     rgb, kind = random_image(rng)
     quality = float(rng.choice([84, 85, 88, 90, 93, 95, 97, 99, 100]))
     lookahead = int(rng.choice([1, 2, 3, 3, 3, 5]))
     new_model = bool(rng.random() < 0.8)
-    rok, rjpeg, rtrace, _, _ = reflib.process_rgb(rgb, quality, lookahead=lookahead, new_zeroing_model=new_model)
+    rok, rjpeg, rtrace, _, _ = ref.process_rgb(rgb, quality, lookahead=lookahead, new_zeroing_model=new_model)
     h, w, _ = rgb.shape
     st = gb.ProcessStats(debug_output=[])
     p = gb.Params(butteraugli_target=gb.butteraugli_score_for_quality(quality, lib=port),
